@@ -5,7 +5,7 @@ One "step" = one frame of the SSGI chain over one batch of synthetic G-buffer pl
   K1 SSGI trace (steps 20 / refine 5) -> K2 temporal reprojection (2 planes) ->
   K3 Poisson denoise x4 (denoiseIterations = 2) -> K4 GI compose          (432 B/px algorithmic, SURVEY.md §8d)
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N = 1 : one 3840x2160 frame per step on one GPU (the configuration the metric is quoted on).
 N > 1 : the SAME 3840x2160 frame, strong scaling: row bands over N ranks (rfx_group_*: halo rows recomputed locally, last frame's
@@ -21,6 +21,10 @@ configs : device time + roofline of the other single-GPU BASELINE configs (C1 mo
 cpu_baseline / --impl reference: the reference's own shaders compiled for the CPU (oracle/_ref, when built) or the CPU restatement in
 oracle/ (the reference's run time is WebGL-only and cannot run here: no GL,
           no JS engine) on the box's host cores, bounded sample, thread count pinned and reported.
+--dump-outputs DIR: after the timed steps, the `composed` plane of the last timed step (what a caller of the chain receives) as
+          DIR/composed.npy, float32.  A plane larger than 64 MB (the 4K frame) is stored as a fixed, seeded sample of its pixels, shape
+          (pixels, 4), the same pixels on every run at that size.  The inputs are synthetic and deterministic, so two builds run with the
+          same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -40,6 +44,7 @@ import numpy as np  # noqa: E402
 
 WIDTH, HEIGHT = 3840, 2160
 DENOISE_ITERATIONS = 2
+DUMP_BYTES, DUMP_SEED = 64_000_000, 20261017  # --dump-outputs: size bound of all files together, seed of the pixel sample
 ALGO_BYTES = {  # SURVEY.md §8(d): algorithmic bytes per output pixel
     "K1_ssgi_trace": 76, "K2_temporal_reproject": 80, "K3_poisson_pass0": 68, "K3_poisson_pass1plus": 52, "K4_gi_compose": 52,
 }
@@ -155,6 +160,23 @@ def chain_options(ch, o, W, H):
         width, height = W, H
 
     return ch.chain_options(_I, o)
+
+
+def dump_outputs(out_dir: str, **planes) -> None:
+    """--dump-outputs: each (H, W, C) plane as <out_dir>/<name>.npy in float32; one over its share of DUMP_BYTES becomes a seeded
+    sample of its pixels (sorted pixel order)"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in planes.items():
+        a = np.asarray(a, np.float32)
+        n = (DUMP_BYTES // len(planes) - 4096) // a[0, 0].nbytes  # pixels that fit the share (less the .npy header)
+        note = ""
+        if a.shape[0] * a.shape[1] > n:
+            px = a.reshape(a.shape[0] * a.shape[1], -1)
+            a = px[np.sort(np.random.default_rng(DUMP_SEED).choice(px.shape[0], n, replace=False))]
+            note = " (seeded pixel sample)"
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a)
+        print(f"bench.py: wrote {path} {a.shape}{note}", file=sys.stderr)
 
 
 def time_frames(stream, render, K):
@@ -321,6 +343,8 @@ def run_single(args):
     prof = chain.get_profile()
     chain.set_profiling(False)
     launches = ctx.launch_count - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, composed=chain.download(0))
     mpx = W * H / 1e6
     value = mpx / (ms_per_step / 1e3)
 
@@ -596,20 +620,20 @@ def run_reference(args):
     o = ch.Opts(denoise_iterations=DENOISE_ITERATIONS)
     sw, sh = (960, 540) if (args.cpu_width, args.cpu_height) == (0, 0) else (args.cpu_width, args.cpu_height)
     K, Wm = args.steps, args.warmup
-    if args.steps == 100:  # the default K is sized for the GPU arm; a CPU step takes ~0.5 s
-        K, Wm = 20, 3
     inp = ch.make_inputs(sw, sh, 2, reference_env=True)
     frames = inp.frames
     cores = int(orc.lib().orc_num_threads())
 
     def step_block(n):
         inp.frames = [frames[i % 2] for i in range(n)]
-        ch.run_oracle_chain(inp, o, capture=("composed",), lean=True, impl=ref)
+        return ch.run_oracle_chain(inp, o, capture=("composed",), lean=True, impl=ref)
 
     step_block(Wm)
     t0 = time.perf_counter()
-    step_block(K)
+    last = step_block(K)[-1]["composed"]
     dt = (time.perf_counter() - t0) / K
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, composed=last)
     v = round(sw * sh / 1e6 / dt, 4)
     line = {"metric": "SSGI+denoise Mpixels/s at 4K", "value": v, "unit": "Mpixels/s", "n_gpus": int(os.environ.get("WORLD_SIZE", "1")), "steps": K, "warmup": Wm,
             "ms_per_step": round(dt * 1e3, 3), "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "impl": "reference",
@@ -625,8 +649,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
-    ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--steps", type=int, help="timed steps (default 100; --impl reference: 20, a CPU step takes ~0.5 s)")
+    ap.add_argument("--warmup", type=int, help="untimed steps before them (default 10; --impl reference: 3)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--width", type=int, default=WIDTH)
     ap.add_argument("--height", type=int, default=HEIGHT)
@@ -635,8 +659,18 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="N = 1: skip the CPU oracle frame (and the parity field computed from it)")
     ap.add_argument("--no-configs", action="store_true", help="N = 1: skip the C1 / C2 / C4 block")
     ap.add_argument("--no-c5", action="store_true", help="N > 1: skip the 7680x4320 measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output of the last timed step to DIR/composed.npy (N = 1 and --impl reference)")
     args = ap.parse_args()
+    cpu = args.impl == "reference"
+    if args.steps is None:
+        args.steps = 20 if cpu else 100
+    if args.warmup is None:
+        args.warmup = 3 if cpu else 10
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
+    if args.dump_outputs and not cpu and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs: the row-sharded run (N > 1) has no single output plane to write")
     if args.impl == "reference":
         run_reference(args)
     elif int(os.environ.get("WORLD_SIZE", "1")) > 1:

@@ -1,5 +1,8 @@
 """CPU tests of the host-side logic that surrounds the kernels: camera math, blue-noise index sequence,
 env-map CDF tables, the synthetic generator's plane layouts."""
+import json
+import os
+
 import numpy as np
 import torch
 
@@ -114,51 +117,29 @@ def test_traa_jitter_r2_sequence_and_view_offset():
     effects.jitter(W, H, object(), 3)  # cameras without setViewOffset are left alone (TAAUtils.js:8)
 
 
-def _js_object(text: str, name: str) -> dict:
-    """the flat `const <name> = { key: literal, ... }` object literal of a reference JS file -> dict (numbers, booleans, strings, null)"""
-    import re
+JS_TABLES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_js_tables.json")
 
-    m = re.search(r"(?:const|let)\s+" + re.escape(name) + r"\s*=\s*\{(.*?)\n\}", text, flags=re.S)
-    assert m, name
-    out = {}
-    for key, val in re.findall(r"^\s*(\w+)\s*:\s*([^,\n/]+?)\s*,?\s*(?://.*)?$", m.group(1), flags=re.M):
-        v = val.strip()
-        if v in ("true", "false"):
-            out[key] = v == "true"
-        elif v == "null":
-            out[key] = None
-        elif v[0] in "\"'":
-            out[key] = v[1:-1]
-        else:
-            try:
-                out[key] = float(v)
-            except ValueError:
-                pass  # an expression (new Color(...), a spread): compared elsewhere
-    return out
+
+def reference_js_tables() -> dict:
+    """the reference's option tables and index exports, as tests/golden/make_golden.py parsed them from its JS files"""
+    with open(JS_TABLES, encoding="utf-8") as f:
+        return json.load(f)
 
 
 def test_option_defaults_equal_the_reference_js_tables():
     """the option tables of effects.py and js/index.js against the reference's own files (SSGIOptions.js, TemporalReprojectPass.js,
-    PoissonDenoisePass.js, AOEffect.js, MotionBlurEffect.js), parsed from the checkout when it is there"""
-    import os
+    PoissonDenoisePass.js, AOEffect.js, MotionBlurEffect.js)"""
     import re
 
-    import pytest
-
-    ref = os.environ.get("RFX_REFERENCE_DIR", "/root/reference")
-    if not os.path.isdir(os.path.join(ref, "src")):
-        pytest.skip("reference checkout absent")
     from realism_effects_b200 import effects
 
-    rd = lambda rel: open(os.path.join(ref, "src", rel), encoding="utf-8").read()  # noqa: E731
-    tables = [("ssgi/SSGIOptions.js", "defaultSSGIOptions", effects.defaultSSGIOptions),
-              ("temporal-reproject/TemporalReprojectPass.js", "defaultTemporalReprojectPassOptions", effects.defaultTemporalReprojectPassOptions),
-              ("denoise/pass/PoissonDenoisePass.js", "defaultPoissonBlurOptions", effects.defaultPoissonBlurOptions),
-              ("ao/AOEffect.js", "defaultAOOptions", effects.defaultAOOptions)]
+    ref = reference_js_tables()
+    tables = [("defaultSSGIOptions", effects.defaultSSGIOptions), ("defaultTemporalReprojectPassOptions", effects.defaultTemporalReprojectPassOptions),
+              ("defaultPoissonBlurOptions", effects.defaultPoissonBlurOptions), ("defaultAOOptions", effects.defaultAOOptions)]
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     js = open(os.path.join(root, "js", "index.js"), encoding="utf-8").read()
-    for rel, name, mine in tables:
-        want = _js_object(rd(rel), name)
+    for name, mine in tables:
+        want = ref[name]
         assert len(want) >= 5, (name, want)
         for k, v in want.items():
             assert k in mine, (name, k)
@@ -173,22 +154,14 @@ def test_option_defaults_equal_the_reference_js_tables():
                 assert re.search(r"\b" + k + r":\s*" + re.escape(("%g" % v)) + r"\b", m.group(1)), (name, k, v)
             else:
                 assert re.search(r"\b" + k + r":\s*" + re.escape(lit), m.group(1)), (name, k, v)
-    mb = re.search(r"const defaultOptions = \{([^}]*)\}", rd("motion-blur/MotionBlurEffect.js")).group(1)
-    assert {k: float(v) for k, v in re.findall(r"(\w+):\s*([\d.]+)", mb)} == {k: float(v) for k, v in effects.defaultMotionBlurOptions.items()}
+    assert ref["MotionBlurEffect.defaultOptions"] == {k: float(v) for k, v in effects.defaultMotionBlurOptions.items()}
 
 
 def test_plugin_surface_exports_every_class_of_the_reference_index():
     """src/index.js:16-31 exports 14 names; effects.py and js/index.js carry all of them (the compute behind each is an rfx_* entry point)"""
-    import os
     import re
 
-    import pytest
-
-    ref = os.environ.get("RFX_REFERENCE_DIR", "/root/reference")
-    idx = os.path.join(ref, "src", "index.js")
-    if not os.path.isfile(idx):
-        pytest.skip("reference checkout absent")
-    names = set(re.findall(r"^\s*(\w+),?\s*$", re.search(r"export \{(.*?)\}", open(idx, encoding="utf-8").read(), flags=re.S).group(1), flags=re.M))
+    names = set(reference_js_tables()["index.js exports"])
     assert len(names) == 14
     from realism_effects_b200 import effects
 

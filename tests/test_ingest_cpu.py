@@ -1,12 +1,11 @@
 """G-buffer ingest (SURVEY.md §8f row 2): the oracle's orc_gbuffer_ingest against (a) the torch restatement of the reference's packers
 in realism_effects_b200/synth.py on identical inputs and (b) the reference's own packGBuffer / packNormal GLSL
-(src/gbuffer/shader/gbuffer_packing.glsl) run through the GLSL runtime."""
+(src/gbuffer/shader/gbuffer_packing.glsl) run through the GLSL runtime, stored as digests."""
 import numpy as np
-import pytest
 import torch
 
 import orc
-import refglsl
+import refpin
 from realism_effects_b200 import synth
 
 
@@ -49,34 +48,27 @@ def test_ingest_options_and_formats():
     assert (gb_b[bg] == np.array([0, 0, 0, 1], np.float32)).all() and (vel_b[bg] == np.array([0, 0, 0, 1], np.float32)).all()
 
 
-GLSL_INGEST = """
-uniform sampler2D tAlbedo; uniform sampler2D tNormal; uniform sampler2D tMaterial; uniform sampler2D tEmissive;
-layout(location = 0) out vec4 oG;
-layout(location = 1) out vec4 oN;
-%s
-void main() {
-  vec4 m = textureLod(tMaterial, vUv, 0.);
-  vec3 n = textureLod(tNormal, vUv, 0.).xyz;
-  oG = packGBuffer(textureLod(tAlbedo, vUv, 0.), n, m.r, m.g, textureLod(tEmissive, vUv, 0.).rgb);
-  oN = vec4(packNormal(n), 0., 0., 1.);
-}
-"""
+def packer_words(gbuffer, normal_word, fg, lit):
+    """the words the ingest shares with the reference's packGBuffer / packNormal: diffuse, normal, roughness/metalness on the foreground,
+    the RGBE8 emissive word where the shader's path is defined (`lit`), and the packed normal of the velocity plane"""
+    return gbuffer[fg][:, :3].view(np.uint32), gbuffer[lit][:, 3].view(np.uint32), normal_word[fg].view(np.uint32)
 
 
-@pytest.mark.skipif(not refglsl.assemble.available(), reason="needs the reference checkout (the packers are read from it)")
-def test_oracle_ingest_equals_the_reference_packgbuffer_glsl():
+def ingest_probe_inputs():
+    """-> frame, SoA planes, foreground and lit masks, digest of the planes the packers read"""
     fr, s = soa_frame()
-    H, W = fr.depth.shape
-    glsl = "varying vec2 vUv;\n" + GLSL_INGEST % refglsl.assemble.read("gbuffer/shader/gbuffer_packing.glsl")
-    sh = refglsl.Shader("ingest_probe", glsl=glsl)
-    sh.tex("tAlbedo", s["albedo"], refglsl.F_RGBA8)
-    sh.tex("tNormal", s["normal"], refglsl.F_RGBA32F)
-    sh.tex("tMaterial", s["material"], refglsl.F_RGBA16F)
-    sh.tex("tEmissive", s["emissive"], refglsl.F_RGBA16F)
-    ref_g, ref_n = sh.run(W, H, [(refglsl.F_RGBA32F, None), (refglsl.F_RGBA32F, None)])
-    gb, vel = orc.gbuffer_ingest(s["albedo"], s["normal"], s["material"], s["emissive"], s["motion"], fr.depth.numpy(), normalize_normals=False)
-    fg = fr.depth.numpy() < 1.0
-    assert (gb[fg][:, :3].view(np.uint32) == ref_g[fg][:, :3].view(np.uint32)).all()               # diffuse, normal, roughness/metalness words
+    depth = fr.depth.numpy()
+    fg = depth < 1.0
     lit = fg & (s["emissive"][..., :3].astype(np.float32).max(-1) > 0)
-    assert lit.any() and (gb[lit][:, 3].view(np.uint32) == ref_g[lit][:, 3].view(np.uint32)).all()  # RGBE8 emissive word where the shader's path is defined
-    assert (vel[fg][:, 2].view(np.uint32) == ref_n[fg][:, 0].view(np.uint32)).all()                # packNormal
+    return fr, s, fg, lit, refpin.digest(s["albedo"], s["normal"], s["material"], s["emissive"], depth)
+
+
+def test_oracle_ingest_equals_the_reference_packgbuffer_glsl():
+    """against the outputs of the reference's gbuffer_packing.glsl run through the GLSL runtime (stored as digests by tests/golden/make_golden.py)"""
+    fr, s, fg, lit, inputs = ingest_probe_inputs()
+    want = refpin.load("ingest_packgbuffer")
+    assert inputs == want["inputs"], "not the inputs the reference's packers were run on"
+    gb, vel = orc.gbuffer_ingest(s["albedo"], s["normal"], s["material"], s["emissive"], s["motion"], fr.depth.numpy(), normalize_normals=False)
+    assert lit.any()
+    got = [refpin.digest(w) for w in packer_words(gb, vel[..., 2], fg, lit)]
+    assert got == want["words"], "diffuse/normal/roughness-metalness, emissive, packNormal words vs the reference: " + str([g == w for g, w in zip(got, want["words"])])

@@ -4,9 +4,9 @@ that executes them (oracle/ref/glsl_rt.h + oracle/ref/transpile.py).
 * runtime tests: small GLSL programs written here whose results are known in closed form — they check the language semantics the
   reference shaders rely on (swizzle l-values, inout copy-back, array constructors, uint arithmetic, quad derivatives with
   helper lanes, discard / early return, sampler state).  They need only g++.
-* pinning tests: the oracle must equal the reference shaders BIT FOR BIT.  They build the shaders from the reference checkout when
-  it is there (this container) and otherwise use the libraries __graft_entry__.build() left in oracle/_ref/ (the GPU box); with
-  neither they are skipped — tests/test_oracle_chain_cpu.py then still checks the oracle against the committed reference outputs.
+* pinning tests: the oracle must equal the reference shaders BIT FOR BIT, in every output of every pass call.  The reference's runs
+  are stored as digests (tests/refpin.py, tests/golden/reference_pins.json, minted by tests/golden/make_golden.py), so these tests
+  need no reference checkout.
 """
 import numpy as np
 import pytest
@@ -14,6 +14,7 @@ import pytest
 import chain_harness as ch
 import orc
 import refglsl
+import refpin
 from realism_effects_b200 import abi
 
 F32, F16 = refglsl.F_RGBA32F, refglsl.F_RGBA16F
@@ -95,70 +96,106 @@ def test_runtime_sampler_state_and_null_sampler():
 
 
 needs_ref = pytest.mark.skipif(not refglsl.available(), reason="neither the reference checkout nor prebuilt oracle/_ref libraries")
-needs_checkout = pytest.mark.skipif(not refglsl.assemble.available(), reason="builds shader variants outside the prebuilt set: needs the reference checkout")
 
 
 def bits(a):
     return np.ascontiguousarray(a).tobytes()
 
 
-@needs_ref
-@pytest.mark.parametrize("mode", [abi.MODE_SSGI, abi.MODE_SSR])
-def test_oracle_equals_reference_shaders_chain(mode):
-    """K1 -> K2 -> K3 x2 -> K4 with history over 3 frames, default options: every plane of every frame, bit for bit"""
-    o = ch.Opts(mode=mode)
-    inp = ch.make_inputs(80, 45, 3)
-    planes = ("ssgi", "tr0", "tr1", "dn0", "dn1", "composed") if mode == abi.MODE_SSGI else ("ssgi", "tr0", "dn0", "composed")
-    a = ch.run_oracle_chain(inp, o, capture=planes, lean=True)
-    b = ch.run_oracle_chain(inp, o, capture=planes, lean=True, impl=refglsl)
-    for t in range(3):
-        for k in planes:
-            assert bits(a[t][k]) == bits(b[t][k]), (t, k, ch.compare(a[t][k], b[t][k], packed=(k == "ssgi" and mode == abi.MODE_SSGI)))
-    assert float(np.abs(b[2]["composed"]).max()) > 0.1  # the comparison is not of empty planes
+# ---- pinning cases: pass sequences run on the reference's shaders by tests/golden/make_golden.py (refpin.Record) and on the oracle by the
+# tests below (refpin.Replay); `m` executes the passes
+def chain_case(m, mode):
+    """K1 -> K2 -> K3 x2 -> K4 with history over 3 frames, default options"""
+    return ch.run_oracle_chain(ch.make_inputs(80, 45, 3), ch.Opts(mode=mode), capture=("composed",), lean=True, impl=m)
 
 
-@needs_ref
-def test_oracle_equals_reference_shaders_effect_passes():
+def effect_passes_case(m):
     """K5 (fog), K6 + AO denoise + K7, K8, TRAA K2 + K9"""
     inp = ch.make_inputs(64, 36, 2)
     f0, f1 = inp.frames
     H, W = f1["depth"].shape
-    z = np.zeros((H, W, 4), np.float16)
-    hp = ch.hbao_params(f1["cam"], 991)
-    ao_o, ao_r = orc.hbao(hp, f1["depth"], inp.blue, z), refglsl.hbao(hp, f1["depth"], inp.blue, z)
-    assert bits(ao_o) == bits(ao_r) and float(ao_r[..., 3].astype(np.float32).min()) < 0.99
-    for x, y in zip(ch.ao_denoise(orc, f1, inp.blue, ao_o), ch.ao_denoise(refglsl, f1, inp.blue, ao_r)):
-        assert bits(x) == bits(y)
-    assert bits(orc.ao_compose(ch.ao_compose_params(), f1["depth"], ao_o, f1["direct"])) == bits(refglsl.ao_compose(ch.ao_compose_params(), f1["depth"], ao_r, f1["direct"]))
-    for x, y in zip(ch.traa_two_frames(orc, f0, f1), ch.traa_two_frames(refglsl, f0, f1)):
-        assert bits(x) == bits(y)
-    assert bits(orc.traa_compose(f1["direct"])) == bits(refglsl.traa_compose(f1["direct"]))
-    vel = ch.rotation_velocity_field(W, H, f1["depth"])
-    mp = ch.motion_blur_params(W, H, frame=7)
-    assert bits(orc.motion_blur(mp, vel, f1["direct"], inp.blue)) == bits(refglsl.motion_blur(mp, vel, f1["direct"], inp.blue))
+    ao = m.hbao(ch.hbao_params(f1["cam"], 991), f1["depth"], inp.blue, np.zeros((H, W, 4), np.float16))
+    ch.ao_denoise(m, f1, inp.blue, ao)
+    m.ao_compose(ch.ao_compose_params(), f1["depth"], ao, f1["direct"])
+    ch.traa_two_frames(m, f0, f1)
+    m.traa_compose(f1["direct"])
+    m.motion_blur(ch.motion_blur_params(W, H, frame=7), ch.rotation_velocity_field(W, H, f1["depth"]), f1["direct"], inp.blue)
     gi = np.random.default_rng(5).uniform(0, 2, (H, W, 4)).astype(np.float32)
     for exp2 in (False, True):
-        fp = ch.fog_params(f1["cam"], exp2)
-        assert bits(orc.ssgi_compose(f1["depth"], gi, f1["direct"], fp)) == bits(refglsl.ssgi_compose(f1["depth"], gi, f1["direct"], fp))
-    assert bits(orc.ssgi_compose(f1["depth"], gi, f1["direct"])) == bits(refglsl.ssgi_compose(f1["depth"], gi, f1["direct"]))
+        m.ssgi_compose(f1["depth"], gi, f1["direct"], ch.fog_params(f1["cam"], exp2))
+    m.ssgi_compose(f1["depth"], gi, f1["direct"])
+    return ao
 
 
-@needs_ref
-def test_oracle_equals_reference_shaders_cosmetic_effects_and_taa():
+def cosmetic_case(m):
     """SharpnessEffect / LensDistortionEffect / GradualBackgroundEffect / SparkleEffect alone and merged in EffectPass order, and TAAPass"""
     inp = ch.make_inputs(96, 54, 2)
     f1 = inp.frames[1]
-    for effs, sp in ch.FX_CASES:
-        p = ch.fx_params(f1["cam"], effs, sp)
-        a, b = orc.effects(p, f1["direct"], f1["depth"], f1["velocity"]), refglsl.effects(p, f1["direct"], f1["depth"], f1["velocity"])
-        assert bits(a) == bits(b), (effs, sp)
+    outs = [m.effects(ch.fx_params(f1["cam"], effs, sp), f1["direct"], f1["depth"], f1["velocity"]) for effs, sp in ch.FX_CASES]
+    hist = np.random.default_rng(1).integers(0, 256, (54, 96, 4), dtype=np.uint8)
+    for p in ch.taa_cases():
+        m.taa(p, f1["direct"], hist)
+    return inp, outs
+
+
+def orthographic_case(m, mode):
+    """the `#else` branches of PERSPECTIVE_CAMERA (K1 ray set-up, getViewZ, the view directions of K2 and K4) through a three.js OrthographicCamera"""
+    inp = ch.make_inputs(64, 40, 2, orthographic=True)
+    return inp, ch.run_oracle_chain(inp, ch.Opts(mode=mode), capture=("composed",), lean=True, impl=m)
+
+
+def random_option_sets_case(m):
+    """tools/fuzz_pin.py in small: random uniform values, shader variants, frame sizes (odd, portrait) and camera motion, through the chain and
+    each single pass"""
+    import os
+    import sys
+
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
+    import fuzz_pin
+
+    rng = np.random.default_rng(20260923)
+    for _ in range(4):
+        n, bad = fuzz_pin.run_chain(*fuzz_pin.draw_chain(rng), ref=m)
+        assert n > 0 and not bad, bad
+    n, bad = fuzz_pin.run_passes(rng, ref=m)
+    assert n == 11 and not bad, bad
+
+
+PINNED = {  # case name in tests/golden/reference_pins.json -> pass sequence
+    **{f"chain_mode{mode}": (lambda m, mode=mode: chain_case(m, mode)) for mode in (abi.MODE_SSGI, abi.MODE_SSR)},
+    "effect_passes": effect_passes_case,
+    "cosmetic_effects_and_taa": cosmetic_case,
+    **{f"orthographic_mode{mode}": (lambda m, mode=mode: orthographic_case(m, mode)) for mode in (abi.MODE_SSGI, abi.MODE_SSR)},
+    "random_option_sets": random_option_sets_case,
+}
+
+
+@pytest.mark.parametrize("mode", [abi.MODE_SSGI, abi.MODE_SSR])
+def test_oracle_equals_reference_shaders_chain(mode):
+    """every pass of every frame, bit for bit"""
+    pin = refpin.Replay(f"chain_mode{mode}")
+    out = chain_case(pin, mode)
+    pin.finish()
+    assert float(np.abs(out[2]["composed"]).max()) > 0.1  # the comparison is not of empty planes
+
+
+def test_oracle_equals_reference_shaders_effect_passes():
+    pin = refpin.Replay("effect_passes")
+    ao = effect_passes_case(pin)
+    pin.finish()
+    assert float(ao[..., 3].astype(np.float32).min()) < 0.99
+
+
+def test_oracle_equals_reference_shaders_cosmetic_effects_and_taa():
+    pin = refpin.Replay("cosmetic_effects_and_taa")
+    inp, outs = cosmetic_case(pin)
+    pin.finish()
+    f1 = inp.frames[1]
+    for (effs, sp), a in zip(ch.FX_CASES, outs):
         if effs != [abi.FX_SPARKLE] or sp:  # (with the reference's orthographic getViewZ branch the sparkle term underflows on this scene)
             assert bits(a) != bits(f1["direct"])  # the effect does something
     fade = orc.effects(ch.fx_params(f1["cam"], [abi.FX_GRADUAL_BACKGROUND]), f1["direct"], f1["depth"], f1["velocity"]).astype(np.float32)
     assert len(np.unique(fade[..., 0])) > 50       # the blend towards the background colour is exercised, not saturated
-    hist = np.random.default_rng(1).integers(0, 256, (54, 96, 4), dtype=np.uint8)
-    for p in ch.taa_cases():
-        assert bits(orc.taa(p, f1["direct"], hist)) == bits(refglsl.taa(p, f1["direct"], hist))
 
 
 @needs_ref
@@ -180,37 +217,20 @@ def test_prebuilt_reference_shaders_run_without_the_checkout():
     assert r.returncode == 0 and "ok" in r.stdout, r.stdout + r.stderr
 
 
-@needs_checkout
 @pytest.mark.parametrize("mode", [abi.MODE_SSGI, abi.MODE_SSR])
 def test_oracle_equals_reference_shaders_orthographic_camera(mode):
-    """the `#else` branches of PERSPECTIVE_CAMERA (K1 ray set-up, getViewZ, the view directions of K2 and K4) through a three.js OrthographicCamera"""
-    inp = ch.make_inputs(64, 40, 2, orthographic=True)
+    pin = refpin.Replay(f"orthographic_mode{mode}")
+    inp, a = orthographic_case(pin, mode)
+    pin.finish()
     assert inp.frames[0]["cam"]["perspective"] is False and abi.make_camera(inp.frames[0]["cam"]).perspective == 0
-    o = ch.Opts(mode=mode)
-    planes = ("ssgi", "tr0", "dn0", "composed")
-    a = ch.run_oracle_chain(inp, o, capture=planes, lean=True)
-    b = ch.run_oracle_chain(inp, o, capture=planes, lean=True, impl=refglsl)
-    for f in range(2):
-        for k in planes:
-            assert bits(a[f][k]) == bits(b[f][k]), (f, k)
-    assert float(np.abs(np.asarray(b[1]["composed"], np.float32)).max()) > 0.1
+    assert float(np.abs(np.asarray(a[1]["composed"], np.float32)).max()) > 0.1
     p = ch.Opts()  # and it is a different image from the perspective one on the same planes
     assert bits(ch.run_oracle_chain(ch.make_inputs(64, 40, 1), p, capture=("composed",), lean=True)[0]["composed"]) != bits(a[0]["composed"])
 
 
-@needs_checkout
 def test_random_option_sets_oracle_equals_reference_shaders():
-    """tools/fuzz_pin.py in small: random uniform values, shader variants, frame sizes (odd, portrait) and camera motion; every plane of the chain and of
-    each single pass must be bit-equal between the oracle and the reference's shaders (profiles/r02_fuzz_pin_seed*.json: 460 cases, 0 differing pixels)"""
-    import os
-    import sys
-
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
-    import fuzz_pin
-
-    rng = np.random.default_rng(20260923)
-    for _ in range(4):
-        n, bad = fuzz_pin.run_chain(*fuzz_pin.draw_chain(rng))
-        assert n > 0 and not bad, bad
-    n, bad = fuzz_pin.run_passes(rng)
-    assert n == 11 and not bad, bad
+    """every plane of the chain and of each single pass bit-equal between the oracle and the reference's shaders
+    (profiles/r02_fuzz_pin_seed*.json: 460 cases, 0 differing pixels)"""
+    pin = refpin.Replay("random_option_sets")
+    random_option_sets_case(pin)
+    pin.finish()

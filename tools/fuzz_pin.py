@@ -51,14 +51,14 @@ def draw_chain(rng) -> tuple:
     return W, H, F, okw, ikw
 
 
-def run_chain(W, H, F, okw, ikw):
+def run_chain(W, H, F, okw, ikw, ref=refglsl):
     o = ch.Opts(**okw)
     inp = ch.make_inputs(W, H, F, **ikw)
     planes = [p for p in PLANES if not (o.mode == abi.MODE_SSR and p in ("tr1", "dn1")) and not (o.denoise_mode != 0 and p in ("dn0", "dn1"))]
     if o.denoise_mode == 2:
         planes = [p for p in planes if p != "composed"]
     a = ch.run_oracle_chain(inp, o, capture=planes, lean=True)
-    b = ch.run_oracle_chain(inp, o, capture=planes, lean=True, impl=refglsl)
+    b = ch.run_oracle_chain(inp, o, capture=planes, lean=True, impl=ref)
     bad = {}
     for f, (x, y) in enumerate(zip(a, b)):
         for k in planes:
@@ -68,8 +68,9 @@ def run_chain(W, H, F, okw, ikw):
     return len(planes) * F, bad
 
 
-def run_passes(rng):
-    """one random draw of every single-pass surface; returns (planes compared, {plane: differing pixels})"""
+def run_passes(rng, ref=refglsl):
+    """one random draw of every single-pass surface; returns (planes compared, {plane: differing pixels}).  `ref`: what the oracle is
+    compared with (the reference's shaders, or tests/refpin.py's record / replay of them)"""
     W, H = int(rng.choice([40, 64, 96])), int(rng.choice([30, 54, 77]))
     ortho = bool(rng.random() < 0.3)
     inp = ch.make_inputs(W, H, 2, fov=float(rng.uniform(30.0, 75.0)), orthographic=ortho)
@@ -79,7 +80,7 @@ def run_passes(rng):
 
     def both(tag, fn):
         nonlocal n
-        for i, (x, y) in enumerate(zip(fn(orc), fn(refglsl))):
+        for i, (x, y) in enumerate(zip(fn(orc), fn(ref))):
             n += 1
             d = diff(x, y)
             if d["n_px"]:
